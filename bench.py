@@ -3,6 +3,7 @@
 3 source views, 18 keypoints).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config {2,3,4,5}] [--scene {ones,hull}] [--impl reference]
+                    [--dump-outputs DIR]
 
 A step = one pass of the hot path over one synthetic frame: re-layout of the (new) source feature
 maps + ray generation + sampling + shading + compositing for every pixel of the novel view.
@@ -21,6 +22,10 @@ The frames are exchanged with ONE NCCL all-gather.
             measured live (valid-sample counter of the launch, CUDA events around the kernel on the launch stream inside the
             timed region), against the measured dense bf16 tensor peak in MEASURED_PEAKS.json; `pair` adds the colour kernel
             (executed FLOPs: 419 200 per valid sample + 79 536 per sample with density > 0).
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the render of the last timed step returned (every output plane
+            of its frame, and with N > 1 ranks the all-gathered frames) as DIR/<name>.npy in float32; should that exceed 64 MB, every
+            array keeps the same fixed, seeded sample of its pixels (the last two axes flattened).  The inputs are generated from
+            fixed seeds, so two builds run with the same arguments can be compared output for output.
 `cpu_baseline` / `--impl reference`: the CPU oracle port (oracle/, torch-CPU, all host threads) on a bounded sample of the
             same workload (a strided pass of the same frame: 4096 rays, fewer when that would take too long).
 """
@@ -223,7 +228,11 @@ def main():
     ap.add_argument("--n-kpt", type=int, default=N_KPT)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         return run_reference_arm(args, cfg, out_fd)
@@ -288,6 +297,8 @@ def main():
             out = D.gather_views(res[key], world)
         if k >= 0:
             gev[k][1].record()
+        if k == args.steps - 1:
+            gstate["res"], gstate["out"] = res, out   # what --dump-outputs writes
         return out
 
     cfgk = dict(sample_per_ray_c=S_c, sample_per_ray_f=S_f, fine=fine, uniform=True, ert_eps=ert)
@@ -330,6 +341,19 @@ def main():
     clocks = sampler.stop()
     st = m.stats()   # counters of the LAST step's render, event times summed over the timed steps
     m.set_profiling(False)
+    if args.dump_outputs and rank == 0:
+        dump = dict(gstate["res"])
+        if world > 1:
+            dump["gathered_" + key] = gstate["out"]
+        limit, total = 64 << 20, sum(v.numel() * 4 for v in dump.values())
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, v in dump.items():
+            a = v.float().cpu().numpy()
+            if total > limit:
+                a = a.reshape(*a.shape[:-2], -1)
+                n = a.shape[-1]
+                a = a[..., np.sort(np.random.default_rng(0).choice(n, n * limit // total, replace=False))]
+            np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
     ms_rank = sum(e0.elapsed_time(e1) for e0, e1 in evs)
     gather_ms = sum(e0.elapsed_time(e1) for e0, e1 in gev)
     mine = torch.tensor([ms_rank, st["shade_ms"], st["geo_ms"], gather_ms, float(st["samples_valid"]), float(st["samples_coloured"])],

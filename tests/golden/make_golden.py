@@ -2,10 +2,14 @@
 
 Run in the build container only (the GPU box has no /root/reference):
     python tests/golden/make_golden.py
-Writes tests/golden/<case>.npz for every entry of CASES (or only the cases named on the command
-line).  Inputs are regenerated from seeds by keypointnerf_b200.synthetic; the .npz files hold the
+Writes tests/golden/<case>.npz for every entry of CASES and dropin_sweep.npz (or only the cases named
+on the command line).  Inputs are regenerated from seeds by keypointnerf_b200.synthetic; the .npz files hold the
 reference's outputs (and, for the tiny cases, per-sample intermediates captured with forward
-hooks), plus an input checksum so that drift in the seeded generators is detected.
+hooks), plus an input checksum so that drift in the seeded generators is detected.  To keep every
+file under 1 MB, per-sample arrays are stored for a fixed, seeded subset: the tiny cases keep every
+valid query point and a sample of the invalid ones (``query_*``, positions ``sel`` of the stage
+intermediates index into that subset); the config-size passes with ``rays`` set keep that many rays
+of the pass (``rays`` = their row-major indices) for ``contrib_coarse``, ``z_coarse`` and ``z_fine``.
 
 Scenes: "hull" = ellipsoid-silhouette foreground masks (every ray's last sample is invalid, so no
 ray sits on the reference's final-sample discontinuity and every ray is compared); "ones" = the
@@ -35,14 +39,26 @@ def _stub(name, **attrs):
     return m
 
 
+class _LightningModule(torch.nn.Module):
+    def save_hyperparameters(self, *a, **k):
+        pass
+
+    def log(self, *a, **k):
+        pass
+
+    @property
+    def device(self):
+        return torch.device("cpu")
+
+
 def import_reference():
     k = _stub("kornia")
-    k.utils = _stub("kornia.utils", tensor_to_image=lambda x: x)
+    k.utils = _stub("kornia.utils", tensor_to_image=lambda x: x.permute(0, 2, 3, 1).cpu().numpy())
     k.metrics = _stub("kornia.metrics")
     kg = _stub("kornia.geometry")
     kg.conversions = _stub("kornia.geometry.conversions", convert_points_to_homogeneous=lambda x: x)
     k.geometry = kg
-    _stub("pytorch_lightning", LightningModule=torch.nn.Module)
+    _stub("pytorch_lightning", LightningModule=_LightningModule)
     _stub("pytorch_lightning.utilities")
     _stub("pytorch_lightning.utilities.apply_func", move_data_to_device=lambda b, d: b)
     _stub("skimage")
@@ -89,7 +105,7 @@ def checksum(scene, weights):
     return h.hexdigest()
 
 
-def run_tile(M, net, scene, target, level, x_off, y_off, S_c, S_f, fine, capture=False, keep=256):
+def run_tile(M, net, scene, target, level, x_off, y_off, S_c, S_f, fine, capture=False, keep=128, keep_pts=None):
     cam, cam_tar, sp_data, feat_geo, feat_tex, img, fg, bounds = ref_inputs(scene, target)
     cap = {}
     hooks = []
@@ -149,25 +165,33 @@ def run_tile(M, net, scene, target, level, x_off, y_off, S_c, S_f, fine, capture
         del net.query
         del net.rgba2out
         N = cap["query_pts"].shape[1]
-        sel = np.linspace(0, N - 1, num=min(keep, N)).astype(np.int64)
+        # stored query points (keep_pts set): every valid one and a seeded sample of the invalid ones (whose outputs are zero)
+        valid = cap["query_valid"][0, :, 0].numpy()
+        pts = np.arange(N)
+        if keep_pts is not None:
+            assert valid.sum() <= keep_pts
+            invalid = np.flatnonzero(~valid)
+            extra = np.random.default_rng(0).choice(invalid, min(len(invalid), keep_pts - int(valid.sum())), replace=False)
+            pts = np.sort(np.concatenate([np.flatnonzero(valid), extra]))
+        sel = np.linspace(0, len(pts) - 1, num=min(keep, len(pts))).astype(np.int64)   # positions in pts
+        at = pts[sel]                                                                  # indices into the N query points
         V = scene["n_views"]
         res["sel"] = sel
-        res["query_pts"] = cap["query_pts"][0].numpy()
-        res["query_view"] = cap["query_view"][0].numpy()
-        res["query_out"] = cap["query_out"][0].numpy()
-        res["query_valid"] = cap["query_valid"][0, :, 0].numpy()
-        res["enc"] = cap["enc"].numpy()[:, sel]                       # (V,sel,7K)
-        res["pw"] = cap["pw"][0].numpy()[:, :, 0]                      # (V,N)
-        res["f64"] = cap["f64"][0].numpy()[:, sel]
-        res["f8"] = cap["f8"][0].numpy()[:, sel]
-        res["x_view"] = cap["x_view"][0].numpy()[:, sel]
-        res["x_pool"] = cap["x_pool"][0].numpy()[sel]
-        res["geo_out"] = cap["geo_out"][0].numpy()
-        R = cap["ibr_rgb"].shape[0]
-        res["ibr_feat"] = cap["ibr_feat"].reshape(N, V, -1).numpy()[sel]      # (sel,V,35)
-        res["ibr_raydiff"] = cap["ibr_raydiff"].reshape(N, V, -1).numpy()[sel]
-        res["ibr_rgb"] = cap["ibr_rgb"].reshape(N, 3).numpy()
-        for k in ("contrib_coarse", "z_coarse", "rgba_coarse", "contrib_fine", "z_fine", "rgba_fine"):
+        res["query_pts"] = cap["query_pts"][0].numpy()[pts]
+        res["query_view"] = cap["query_view"][0].numpy()[pts]
+        res["query_out"] = cap["query_out"][0].numpy()[pts]
+        res["query_valid"] = valid[pts]
+        res["enc"] = cap["enc"].numpy()[:, at]                        # (V,sel,7K)
+        res["pw"] = cap["pw"][0].numpy()[:, pts, 0]                    # (V,pts)
+        res["f64"] = cap["f64"][0].numpy()[:, at]
+        res["f8"] = cap["f8"][0].numpy()[:, at]
+        res["x_view"] = cap["x_view"][0].numpy()[:, at]
+        res["x_pool"] = cap["x_pool"][0].numpy()[at]
+        res["geo_out"] = cap["geo_out"][0].numpy()[pts]
+        res["ibr_feat"] = cap["ibr_feat"].reshape(N, V, -1).numpy()[at]       # (sel,V,35)
+        res["ibr_raydiff"] = cap["ibr_raydiff"].reshape(N, V, -1).numpy()[at]
+        res["ibr_rgb"] = cap["ibr_rgb"].reshape(N, 3).numpy()[pts]
+        for k in ("contrib_coarse", "z_coarse", "rgba_coarse", "z_fine"):
             if k in cap:
                 res[k] = cap[k][0].numpy()
     return res
@@ -176,7 +200,7 @@ def run_tile(M, net, scene, target, level, x_off, y_off, S_c, S_f, fine, capture
 # name -> dict(src, tgt, az, zoom, level, off, S_c, S_f, fine, n_kpt, seeds, fg_mode, fg_hole, capture, keep)
 def _c(**kw):
     d = dict(src_size=512, tgt_size=512, azimuth=1.0, zoom=1.0, level=4, x_off=0, y_off=0, S_c=32, S_f=0, fine=False,
-             n_kpt=18, scene_seed=2, w_seed=26, fg_mode="hull", fg_hole=False, capture="none")
+             n_kpt=18, scene_seed=2, w_seed=26, fg_mode="hull", fg_hole=False, capture="none", rays=None)
     d.update(kw)
     return d
 
@@ -193,10 +217,10 @@ CASES = {
     "cfg1_tile": _c(),
     "cfg1_ones": _c(fg_mode="ones", capture="some"),
     # BASELINE config 2 at config size: one strided pass of the 512x512x128 frame (hull scene and the bench scene)
-    "cfg2_pass": _c(x_off=3, y_off=5, S_c=128, capture="some"),
-    "cfg2_pass_ones": _c(x_off=3, y_off=5, S_c=128, fg_mode="ones", capture="some"),
+    "cfg2_pass": _c(x_off=3, y_off=5, S_c=128, capture="some", rays=1024),
+    "cfg2_pass_ones": _c(x_off=3, y_off=5, S_c=128, fg_mode="ones", capture="some", rays=1024),
     # BASELINE config 3 at config size: 64 coarse + 64 fine
-    "cfg3_pass": _c(x_off=3, y_off=5, S_c=64, S_f=64, fine=True, capture="some"),
+    "cfg3_pass": _c(x_off=3, y_off=5, S_c=64, S_f=64, fine=True, capture="some", rays=1024),
     # BASELINE config 4: 1024^2 target, one level-5 pass (64x64 rays), 128 samples
     "cfg4_pass": _c(tgt_size=1024, level=5, x_off=7, y_off=9, S_c=128),
     # BASELINE config 5: second novel view of the sweep (azimuth 1.0 + pi/4)
@@ -204,12 +228,43 @@ CASES = {
 }
 
 
+def dropin_sweep(M):
+    """dropin_sweep.npz: the reference's KeypointNeRFLightningModule loads a seeded checkpoint with its strict
+    load_state_dict and renders a two-camera sweep through render_novel_views (src/model.py:474-507).  Stores the module's
+    state_dict names and shapes, the checksums of the checkpoint and of the sweep's inputs, and the 8-bit renderings."""
+    from keypointnerf_b200.config import default_cfg
+    from tests.util import seeded_checkpoint, state_dict_checksum, sweep_checksum, sweep_inputs
+    n_kpt, S_c, S_f = 18, 12, 8
+    cfg = default_cfg(n_kpt)
+    cfg["models"]["KeypointNeRF"]["dr_kwargs"].update(sample_per_ray_c=S_c, sample_per_ray_f=S_f)
+    cfg.update(expname="t", out_dir=HERE, training={})
+    ref = M.KeypointNeRFLightningModule(cfg, None).eval()
+    shapes = [(k, list(v.shape)) for k, v in ref.state_dict().items()]
+    sd = seeded_checkpoint(shapes, syn.make_weights(n_kpt))
+    ref.load_state_dict({k: torch.from_numpy(v) for k, v in sd.items()})
+    batch, cams = sweep_inputs(n_kpt)
+    input_sha = sweep_checksum(batch, cams)
+    batch = {k: torch.from_numpy(np.ascontiguousarray(v)) for k, v in batch.items()}
+    cams = [{k: torch.from_numpy(v) if isinstance(v, np.ndarray) else v for k, v in c.items()} for c in cams]
+    with torch.no_grad():
+        want = ref.render_novel_views(cams, batch, only_renderings=True)[0]
+    meta = {"n_kpt": n_kpt, "S_c": S_c, "S_f": S_f, "state_dict": shapes}
+    np.savez_compressed(os.path.join(HERE, "dropin_sweep.npz"), renderings=want,
+                        ckpt_sha256=np.frombuffer(state_dict_checksum(sd).encode(), dtype=np.uint8),
+                        input_sha256=np.frombuffer(input_sha.encode(), dtype=np.uint8),
+                        meta=np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8))
+    print("dropin_sweep", want.shape, want.dtype, "max", int(want.max()), flush=True)
+
+
 def main():
     M = import_reference()
     torch.set_num_threads(8)
-    names = sys.argv[1:] or list(CASES)
+    names = sys.argv[1:] or list(CASES) + ["dropin_sweep"]
     nets = {}
     for name in names:
+        if name == "dropin_sweep":
+            dropin_sweep(M)
+            continue
         c = CASES[name]
         scene = syn.make_scene(src_size=c["src_size"], n_views=3, n_kpt=c["n_kpt"], seed=c["scene_seed"],
                                fg_mode=c["fg_mode"], fg_hole=c["fg_hole"])
@@ -219,15 +274,22 @@ def main():
         if key not in nets:
             nets[key] = build_net(M, c["n_kpt"], weights)
         res = run_tile(M, nets[key], scene, target, level=c["level"], x_off=c["x_off"], y_off=c["y_off"], S_c=c["S_c"],
-                       S_f=c["S_f"], fine=c["fine"], capture=c["capture"] != "none")
+                       S_f=c["S_f"], fine=c["fine"], capture=c["capture"] != "none",
+                       keep_pts=3072 if c["capture"] == "all" else None)
         if c["capture"] == "some":   # outputs + what the compositing / resampling tests need, not the per-sample tensors
             keys = ["tex_fg", "depth", "alpha", "tex_fg_fine", "depth_fine", "alpha_fine", "sdf", "z_fine", "contrib_coarse",
                     "z_coarse"]
             valid_frac = float(res["query_valid"].mean())
             res = {k: res[k] for k in keys if k in res}
+            if c["rays"]:
+                rays = np.sort(np.random.default_rng(0).choice(res["tex_fg"][0, 0].size, c["rays"], replace=False))
+                for k in ("z_fine", "contrib_coarse", "z_coarse"):
+                    if k in res:
+                        res[k] = res[k][rays]
+                res["rays"] = rays
         else:
             valid_frac = float(res["query_valid"].mean()) if "query_valid" in res else float("nan")
-        meta = {k: v for k, v in c.items() if k != "capture"}
+        meta = {k: v for k, v in c.items() if k not in ("capture", "rays")}
         res["input_sha256"] = np.frombuffer(checksum(scene, weights).encode(), dtype=np.uint8)
         res["meta"] = np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8)
         np.savez_compressed(os.path.join(HERE, name + ".npz"), **res)

@@ -1,61 +1,24 @@
-"""Drop-in check against the reference's own caller (needs /root/reference: build container only).
+"""Drop-in check of this ``KeypointNeRF`` as the reference's ``KeypointNeRFLightningModule`` drives it, against the
+reference's own renderings (``tests/golden/dropin_sweep.npz``, written by ``tests/golden/make_golden.py``).
 
-The reference's ``KeypointNeRFLightningModule`` (``src/model.py:28-46``) is instantiated twice from the same config: once with the
-reference's ``KeypointNeRF`` and once with ``keypointnerf_b200.model.KeypointNeRF`` patched in (the one-line change of
-INTEGRATION.md).  The reference's checkpoint is loaded into the second one with the reference's own STRICT ``load_ckpt``
-(``src/model.py:113-117``), then both walk ``render_novel_views`` -> ``attach_im_feat`` -> ``render_full_nerf_image`` ->
-``render_pifu_nerf`` (``src/model.py:453-507``) on the same batch.  There is no GPU here, so the CUDA marcher is replaced by a
-stand-in that answers ``set_scene`` / ``render`` with the CPU oracle: what is under test is everything ABOVE the C ABI -- state_dict
-keys, encoders, feature caching, argument marshalling, output dict -- and the images must agree with the reference's.
+The golden holds the names and shapes of the reference module's ``state_dict``, the checksum of a checkpoint made from seeds
+for exactly those names, the checksum of the sweep's seeded inputs, and the 8-bit renderings of a two-camera sweep that the reference's ``render_novel_views``
+(``src/model.py:474-507``) made with that checkpoint.  Here the same checkpoint goes through a strict ``load_state_dict`` of a
+module that holds this class as ``model`` (what the reference's ``load_ckpt``, ``src/model.py:113-117``, does), and the sweep
+makes the same calls: ``attach_im_feat`` once, then ``render_pifu_nerf`` per camera with the reference's keyword arguments
+(``src/model.py:453-473``), ``tex_fg_fine`` clamped to [0, 1] and scaled to 8 bits.  There is no GPU here, so the CUDA
+marcher is replaced by a stand-in that answers ``set_scene`` / ``render`` with the CPU oracle: what is under test is everything
+ABOVE the C ABI -- state_dict keys, encoders, feature caching, argument marshalling, output dict -- and the images must agree
+with the reference's.
 """
+import json
+import math
 import os
-import sys
-import types
 
 import numpy as np
-import pytest
 import torch
 
-REF = "/root/reference"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="needs the reference checkout (build container only)")
-
-
-def _import_reference():
-    def stub(name, **attrs):
-        m = types.ModuleType(name)
-        m.__dict__.update(attrs)
-        sys.modules[name] = m
-        return m
-
-    class LightningModule(torch.nn.Module):
-        def save_hyperparameters(self, *a, **k):
-            pass
-
-        def log(self, *a, **k):
-            pass
-
-        @property
-        def device(self):
-            return torch.device("cpu")
-
-    k = stub("kornia")
-    k.utils = stub("kornia.utils", tensor_to_image=lambda x: x.permute(0, 2, 3, 1).cpu().numpy())
-    k.metrics = stub("kornia.metrics")
-    kg = stub("kornia.geometry")
-    kg.conversions = stub("kornia.geometry.conversions", convert_points_to_homogeneous=lambda x: x)
-    k.geometry = kg
-    stub("pytorch_lightning", LightningModule=LightningModule)
-    stub("pytorch_lightning.utilities")
-    stub("pytorch_lightning.utilities.apply_func", move_data_to_device=lambda b, d: b)
-    stub("skimage")
-    stub("skimage.metrics", structural_similarity=None)
-    stub("imageio")
-    torch.Tensor.cuda = lambda self, *a, **kw: self
-    if REF not in sys.path:
-        sys.path.insert(0, REF)
-    import src.model as M
-    M.VGGLoss = lambda: None
-    return M
+from tests.util import GOLDEN, seeded_checkpoint, state_dict_checksum, sweep_checksum, sweep_inputs
 
 
 class OracleMarcher:
@@ -92,66 +55,66 @@ class OracleMarcher:
         return res
 
 
-def _batch(scene, tgt):
-    """What ZJUDataset yields for one frame (``src/zju_dataset.py:217-343``): index 0 = target view, 1.. = source views."""
-    V, s = scene["n_views"], scene["src_size"]
-    t = lambda a: torch.from_numpy(np.ascontiguousarray(a))
-    Rt = np.concatenate([tgt["RT"][:, :3, :4], scene["extrin"][:, :3, :4]], 0)[None]
-    Ks = np.concatenate([tgt["K"][:, :3, :3], scene["K"][:, :3, :3]], 0)[None]
-    imgs = np.concatenate([np.zeros((1, 3, s, s), np.float32), scene["img"]], 0)[None]
-    msk = np.concatenate([np.ones((1, 1, s, s), np.float32), scene["fg"].astype(np.float32)], 0)[None]
-    return {"images": t(imgs), "images_masks": t(msk), "Rt": t(Rt), "K": t(Ks), "kpt3d": t(scene["kpt3d"]),
-            "bounds": t(scene["bounds"]), "mask_at_box": torch.ones(1, s * s)}
-
-
-@pytest.fixture
-def keep_tensor_cuda():
-    orig = torch.Tensor.cuda          # the CPU harness makes Tensor.cuda the identity (SURVEY.md Appendix C): undo it afterwards
-    yield
-    torch.Tensor.cuda = orig
-
-
-def test_reference_lightning_module_runs_on_this_class(tmp_path, keep_tensor_cuda):
+def test_novel_view_sweep_matches_reference_renderings(tmp_path):
     from keypointnerf_b200 import synthetic as syn
     from keypointnerf_b200.config import default_cfg
-    from keypointnerf_b200.model import KeypointNeRF as Mine
-    M = _import_reference()
-    RefNet = M.KeypointNeRF
-    torch.manual_seed(0)
-    n_kpt = 18
+    from keypointnerf_b200.model import KeypointNeRF
+    g = np.load(os.path.join(GOLDEN, "dropin_sweep.npz"))
+    meta = json.loads(bytes(g["meta"]).decode())
+    want = g["renderings"]
+    n_kpt = meta["n_kpt"]
     cfg = default_cfg(n_kpt)
-    cfg["models"]["KeypointNeRF"]["dr_kwargs"].update(sample_per_ray_c=12, sample_per_ray_f=8)
-    cfg.update(expname="t", out_dir=str(tmp_path), training={})
-    weights = syn.make_weights(n_kpt)
-    scene = syn.make_scene(src_size=128, n_kpt=n_kpt, fg_mode="hull")
-    tgt = syn.make_target(size=64, azimuth=1.0, zoom=2.0)
-    batch = _batch(scene, tgt)
-    cams = [{"intrinsics": torch.from_numpy(syn.make_target(64, az, zoom=2.0)["K"]),
-             "w2cs": torch.from_numpy(syn.make_target(64, az, zoom=2.0)["RT"][0]), "im_h": 64, "im_w": 64, "znear": 2.0, "zfar": 5.0}
-            for az in (1.0, 2.5)]
-    try:
-        ref = M.KeypointNeRFLightningModule(cfg, None).eval()
-        res = ref.model.load_state_dict({k: torch.from_numpy(np.asarray(v)) for k, v in weights.items()}, strict=False)
-        assert not res.unexpected_keys
-        sd = ref.state_dict()
-        sd["model.vgg_loss.vgg.slice1.0.weight"] = torch.zeros(4)   # the real model owns a frozen VGG19 (src/model.py:608)
-        path = os.path.join(tmp_path, "latest.ckpt")
-        torch.save({"state_dict": sd, "epoch": 3, "global_step": 7}, path)
-        with torch.no_grad():
-            want = ref.render_novel_views(cams, batch, only_renderings=True)[0]
+    cfg["models"]["KeypointNeRF"]["dr_kwargs"].update(sample_per_ray_c=meta["S_c"], sample_per_ray_f=meta["S_f"])
 
-        M.KeypointNeRF = Mine                                        # the one-line change of INTEGRATION.md
-        mine = M.KeypointNeRFLightningModule(cfg, None).eval()
-        assert isinstance(mine.model, Mine)
-        assert set(k for k in mine.state_dict()) == set(k for k in ref.state_dict()), "state_dict keys differ from the reference's"
-        assert mine.load_ckpt(path) == (3, 7)                        # strict load_state_dict inside
-        fake = OracleMarcher({k: v.numpy() for k, v in mine.model.state_dict().items() if not k.startswith(("geo_", "tex_", "sp_"))})
-        mine.model.marcher = lambda: fake
-        with torch.no_grad():
-            got = mine.render_novel_views(cams, batch, only_renderings=True)[0]
-    finally:
-        M.KeypointNeRF = RefNet
-    assert got.shape == want.shape == (2, 64, 64, 3) and got.dtype == np.uint8
+    class Module(torch.nn.Module):   # the reference's LightningModule holds the network as `model`
+        def __init__(self):
+            super().__init__()
+            self.model = KeypointNeRF(cfg)
+
+    mine = Module().eval()
+    shapes = {k: list(v.shape) for k, v in mine.state_dict().items()}
+    ref_shapes = {k: s for k, s in meta["state_dict"]}
+    assert shapes == ref_shapes, f"state_dict differs from the reference's: {sorted(set(shapes.items()) ^ set(ref_shapes.items()))[:8]}"
+    sd = seeded_checkpoint(meta["state_dict"], syn.make_weights(n_kpt))
+    assert state_dict_checksum(sd) == bytes(g["ckpt_sha256"]).decode(), "the seeded checkpoint is not the one the golden was made with"
+    sd["model.vgg_loss.vgg.slice1.0.weight"] = np.zeros(4, np.float32)   # the real model owns a frozen VGG19 (src/model.py:608)
+    path = tmp_path / "latest.ckpt"
+    torch.save({"state_dict": {k: torch.from_numpy(v) for k, v in sd.items()}, "epoch": 3, "global_step": 7}, path)
+    mine.load_state_dict(torch.load(path)["state_dict"])             # strict, as the reference's load_ckpt
+    net = mine.model
+    fake = OracleMarcher({k: v.numpy() for k, v in net.state_dict().items() if not k.startswith(("geo_", "tex_", "sp_"))})
+    net.marcher = lambda: fake
+
+    # the reference's decode_batch (src/model.py:309-409): index 0 of the batch is the target view, 1.. the source views
+    batch, cams = sweep_inputs(n_kpt)
+    assert sweep_checksum(batch, cams) == bytes(g["input_sha256"]).decode(), "seeded inputs drifted from the ones the golden run used"
+    t = lambda a: torch.from_numpy(np.ascontiguousarray(a))
+    im = t(batch["images"][0, 1:])
+    V, s = im.shape[0], im.shape[-1]
+    extrin = torch.eye(4).repeat(V, 1, 1)
+    extrin[:, :3, :4] = t(batch["Rt"][0, 1:])
+    intrin = torch.eye(4).repeat(V, 1, 1)
+    intrin[:, :3, :3] = t(batch["K"][0, 1:])
+    cam = {"KRT": intrin @ extrin, "K": intrin, "Rt": t(batch["Rt"][0, 1:]), "extrin": extrin, "znear": 2.0, "zfar": 5.0,
+           "width": s, "height": s, "nml_scale": 100.0}
+    kpt3d = t(batch["kpt3d"])
+    sp_data = {"extrin": extrin, "kpt3d": kpt3d}
+    dr = net.kwargs["dr_kwargs"]
+    got = []
+    with torch.no_grad():
+        net.attach_im_feat(im)
+        for c in cams:
+            K, RT = t(c["intrinsics"]), t(c["w2cs"])[None]
+            cam_tar = {"K": K, "RT": RT, "KRT": K @ RT, "width": c["im_w"], "height": c["im_h"], "nml_scale": 100.0,
+                       "znear": c["znear"], "zfar": c["zfar"]}
+            out = net.render_pifu_nerf(net=net, img_in=im, cam_in=cam, cam_tar=cam_tar, tar_img=None, sp_data=sp_data,
+                                       objcenter=kpt3d[:, 0, :], fine=dr["fine"], uniform=True, objrad=250., blur=3,
+                                       level=max(0, int(math.log(c["im_h"], 2)) - 5), sample_per_ray_c=dr["sample_per_ray_c"],
+                                       sample_per_ray_f=dr["sample_per_ray_f"], src_foreground_mask=t(batch["images_masks"][:, 1:]),
+                                       bounds=t(batch["bounds"]), mask_at_box=t(batch["mask_at_box"]))
+            got.append(out["tex_fg_fine"].clamp(min=0.0, max=1.0).permute(1, 2, 0).numpy())
+    got = (np.stack(got) * 255.).astype(np.uint8)
+    assert got.shape == want.shape == (2, 64, 64, 3) and want.dtype == np.uint8
     assert fake.scene_binds == 1, "the source-image set must be bound (and encoded) once per sweep, not once per camera"
     d = np.abs(got.astype(np.int32) - want.astype(np.int32))
     assert want.max() > 30, "the test scene renders nothing"

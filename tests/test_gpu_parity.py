@@ -158,6 +158,11 @@ def test_tile_fine_free_running(case, engine):
     assert np.quantile(e, 0.99) < t["q99_fine"]
 
 
+def rays(g):
+    """The rays of a pass whose per-sample arrays the golden stores (tests/golden/make_golden.py): all when it has no `rays`."""
+    return g.get("rays", slice(None))
+
+
 def _golden_case(name):
     g, meta, sha = load_golden(name)
     scene, weights, target = scene_from_meta(meta)
@@ -178,7 +183,7 @@ def test_config_size_pass_matches_reference(name, engine):
     good &= check(rep, "alpha", r["alpha"], g["alpha"][0], ALL, t["alpha"])
     good &= check(rep, "depth", r["depth"], g["depth"][0], ALL, t["depth"])
     if "contrib_coarse" in g:
-        good &= check(rep, "contrib", r["contrib"], g["contrib_coarse"], ALL, t["contrib"])
+        good &= check(rep, "contrib", r["contrib"][rays(g)], g["contrib_coarse"], ALL, t["contrib"])
     p = psnr(r["tex_fg"], g["tex_fg"][0])
     print(f"{name} engine {engine}: " + "; ".join(rep) + f"; psnr (all rays) {p:.1f} dB")
     assert good and p > t["psnr"], rep
@@ -187,20 +192,25 @@ def test_config_size_pass_matches_reference(name, engine):
 @pytest.mark.parametrize("engine", ENGINES)
 def test_cfg3_pass_matches_reference(engine):
     """BASELINE config 3 at config size (64 coarse + 64 fine samples) on one pass: coarse image and compositing weights,
-    the fine image on the reference's own resampled depths (pointwise) and free-running (PSNR + resampled-depth quantile)."""
+    the fine image on the reference's own resampled depths (pointwise, on the rays whose depths the golden stores) and
+    free-running (PSNR over every ray + resampled-depth quantile)."""
     g, meta, scene, weights, target, net = _golden_case("cfg3_pass")
     r = _render_tile(net, meta, scene, target, engine=engine, debug=True)
     t = TOL[engine]
+    sub = rays(g)
+    px = lambda a: a.reshape(*a.shape[:-2], -1)[..., sub]   # (.., h, w) image -> the stored rays
     rep = []
     good = check(rep, "tex_fg", r["tex_fg"], g["tex_fg"][0], ALL, t["rgb"])
-    good &= check(rep, "contrib", r["contrib"], g["contrib_coarse"], ALL, t["contrib"])
+    good &= check(rep, "contrib", r["contrib"][sub], g["contrib_coarse"], ALL, t["contrib"])
     p_free = psnr(r["tex_fg_fine"], g["tex_fg_fine"][0])
-    dz = np.abs(r["z_fine"] - g["z_fine"])
-    r2 = _render_tile(net, meta, scene, target, engine=engine, z_override=torch.from_numpy(g["z_fine"]))
-    good &= check(rep, "tex_fg_fine@ref-z", r2["tex_fg_fine"], g["tex_fg_fine"][0], ALL, t["rgb"])
-    good &= check(rep, "alpha_fine@ref-z", r2["alpha_fine"], g["alpha_fine"][0], ALL, t["alpha"])
-    good &= check(rep, "sdf@ref-z", r2["sdf"], g["sdf"][0], ALL, t["sdf"])
-    p_ref = psnr(r2["tex_fg_fine"], g["tex_fg_fine"][0])
+    dz = np.abs(r["z_fine"][sub] - g["z_fine"])
+    z_ref = r["z_fine"].copy()
+    z_ref[sub] = g["z_fine"]
+    r2 = _render_tile(net, meta, scene, target, engine=engine, z_override=torch.from_numpy(z_ref))
+    good &= check(rep, "tex_fg_fine@ref-z", px(r2["tex_fg_fine"]), px(g["tex_fg_fine"][0]), ALL, t["rgb"])
+    good &= check(rep, "alpha_fine@ref-z", px(r2["alpha_fine"]), px(g["alpha_fine"][0]), ALL, t["alpha"])
+    good &= check(rep, "sdf@ref-z", px(r2["sdf"]), px(g["sdf"][0]), ALL, t["sdf"])
+    p_ref = psnr(px(r2["tex_fg_fine"]), px(g["tex_fg_fine"][0]))
     print(f"cfg3 engine {engine}: " + "; ".join(rep) + f"; fine psnr @ref-z {p_ref:.1f} dB, free-running {p_free:.1f} dB, "
           f"z_fine q99 {np.quantile(dz, 0.99):.2e}")
     assert good and p_ref > t["psnr"] and p_free > 55.0 and np.quantile(dz, 0.99) < 1e-3, rep
@@ -217,7 +227,7 @@ def test_bench_scene_pass_matches_reference(name, engine):
     r = _render_tile(net, meta, scene, target, engine=engine, debug=True)
     t = TOL[engine]
     rep = []
-    good = check(rep, "contrib[:, :-1]", r["contrib"][:, :-1], g["contrib_coarse"][:, :-1], ALL, t["contrib"])
+    good = check(rep, "contrib[:, :-1]", r["contrib"][rays(g), :-1], g["contrib_coarse"][:, :-1], ALL, t["contrib"])
     e = np.abs(r["tex_fg"] - g["tex_fg"][0]).max(0)
     frac = float((e > t["rgb"]).mean())
     p = psnr(r["tex_fg"], g["tex_fg"][0])
